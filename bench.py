@@ -4,6 +4,7 @@ N > 1), the reference's own CPU path beside it.
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W   # the reference's own AVX CPU path (rank 0 only)
+    python bench.py ... --dump-outputs DIR   # also write what the last timed step returned as DIR/*.npy (same inputs every run)
 
 A "step" is one decode token of the synthetic Llama-3-8B (random AWQ-INT4 weights in the reference's QM_CUDA layout, random-filled
 fp16 KV cache).  The K timed steps are spread evenly over context lengths 1 -> max_ctx, so ms_per_step estimates the mean cost per
@@ -503,7 +504,18 @@ def run_extras(ctx, dev, stream, peaks):
 # ------------------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, arrays, rank: int, world: int):
+    """--dump-outputs: one DIR/<name>.npy per array (float32 / float64); with N > 1 every rank writes its own, suffixed _rank<r>."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def run_ours(args):
+    import numpy as np
     import torch
     import torch.distributed as dist
 
@@ -521,6 +533,7 @@ def run_ours(args):
     stream = torch.cuda.Stream(dev)
     tp = world > 1 and args.parallel == "tp"
     extra = {}
+    outs = {} if args.dump_outputs else None
     with torch.cuda.stream(stream):
         ctx = Context(local_rank, stream)
         K, W = args.steps, args.warmup
@@ -538,13 +551,16 @@ def run_ours(args):
             torch.cuda.synchronize(dev)
 
         def fill_cache(m, g):
-            # random-filled KV cache so every context length is "already generated"
+            # random-filled KV cache so every context length is "already generated"; seeded so that every run decodes the same inputs
+            gen = torch.Generator(device=dev)
+            gen.manual_seed(4321)
             for l in range(g.num_layers):
-                m.kv_cache(l, 0).normal_(0, 0.5)
-                m.kv_cache(l, 1).normal_(0, 0.5)
+                m.kv_cache(l, 0).normal_(0, 0.5, generator=gen)
+                m.kv_cache(l, 1).normal_(0, 0.5, generator=gen)
 
-        def timed(m, vocab_local):
-            """(device-resident ms, host entry point ms, clocks) over the K timed steps of model m"""
+        def timed(m, vocab_local, outs=None):
+            """(device-resident ms, host entry point ms, clocks) over the K timed steps of model m; `outs` (a dict) receives what the last
+            step of each entry point returned: the device logits of tce_llama_decode, the host logits and greedy token of tce_llama_decode_host"""
             tokpos_all = torch.tensor(list(zip(toks, pos_list)), dtype=torch.int32, device=dev)
             tokpos = torch.zeros(2, dtype=torch.int32, device=dev)
             logits_pinned = torch.empty(vocab_local, dtype=torch.float32).pin_memory()
@@ -561,15 +577,20 @@ def run_ours(args):
                 e1.record(stream)
                 barrier()
             ms_dev = e0.elapsed_time(e1)
+            if outs is not None:
+                outs["logits"] = m.logits().cpu().numpy()
             for i in range(W):
                 m.decode_host(toks[i], pos_list[i], logits_pinned)
             barrier()
             e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e2.record(stream)
             for i in range(W, W + K):
-                m.decode_host(toks[i], pos_list[i], logits_pinned)
+                nxt = m.decode_host(toks[i], pos_list[i], logits_pinned)
             e3.record(stream)
             barrier()
+            if outs is not None:
+                outs["e2e_logits"] = logits_pinned.numpy().copy()
+                outs["e2e_next_token"] = np.array([nxt], dtype=np.float64)
             return ms_dev, e2.elapsed_time(e3), clk.summary()
 
         if tp:
@@ -600,7 +621,7 @@ def run_ours(args):
                 extra["tp_parity_rel_err"] = parity
                 extra["tp_parity_note"] = "max |logits_tp - logits_1gpu| / max |logits_1gpu| over 4 decode steps of the same weights (rank 0 runs the single-GPU model)"
             fill_cache(model, gl)
-            ms_dev, ms_e2e, clocks = timed(model, gl.vocab_size)
+            ms_dev, ms_e2e, clocks = timed(model, gl.vocab_size, outs)
             if args.replicas_too:
                 fill_cache(single, geom)
                 r_dev, _, _ = timed(single, geom.vocab_size)
@@ -614,9 +635,11 @@ def run_ours(args):
             gl = geom
             model = LL.LlamaModel(ctx, geom, max_ctx=args.max_ctx, seed=1234 + rank)
             fill_cache(model, geom)
-            ms_dev, ms_e2e, clocks = timed(model, geom.vocab_size)
+            ms_dev, ms_e2e, clocks = timed(model, geom.vocab_size, outs)
             vocab_local = geom.vocab_size
         kernels_per_step = model.kernels_per_step
+        if outs is not None:
+            dump_outputs(args.dump_outputs, outs, rank, world)
         if rank == 0 and world == 1 and not args.no_extras:
             peaks, _, _ = load_peaks()
             try:
@@ -719,7 +742,7 @@ def run_ours(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=128)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 128; 8 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--model", default="llama3-8b")
@@ -733,17 +756,25 @@ def main():
     # sequence per GPU (no data-path collective, weak scaling), also reported as `replicas_tok_s` beside the tensor-parallel value
     ap.add_argument("--parallel", default="tp", choices=["tp", "replicas"])
     ap.add_argument("--no-replicas", dest="replicas_too", action="store_false", help="N>1 tp: skip the secondary replicas measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (logits, greedy token) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of this project's decode step; the reference arm times bare linears")
     if args.warmup < 3:
         args.warmup = 3
     if args.probe_threads:
         probe_threads(args)
         return
     if args.impl == "reference":
-        if args.steps == 128:
+        if args.steps is None:
             args.steps = 8  # a full token costs seconds on the host: keep the default invocation within minutes
         run_reference(args)
     else:
+        if args.steps is None:
+            args.steps = 128
         run_ours(args)
 
 

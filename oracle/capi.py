@@ -23,8 +23,10 @@ _i32p = np.ctypeslib.ndpointer(np.int32, flags="C_CONTIGUOUS")
 
 
 def build(ref: bool = True) -> None:
-    """(Re)build the oracle .so (and oracle/_ref when /root/reference is present)."""
-    targets = ["oracle"] + (["ref"] if ref else [])
+    """(Re)build the oracle .so and, with ref, oracle/_ref.  oracle/Makefile builds and rebuilds oracle/_ref from the reference tree
+    (its REF, or TCE_REFERENCE_DIR when set) wherever that tree is readable, and leaves it alone elsewhere."""
+    tree = os.environ.get("TCE_REFERENCE_DIR")
+    targets = ["oracle"] + (["ref"] + ([f"REF={tree}"] if tree else []) if ref else [])
     subprocess.run(["make", "-s", "-C", str(HERE)] + targets, check=True)
 
 

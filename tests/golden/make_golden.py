@@ -1,15 +1,23 @@
 #!/usr/bin/env python
-"""Generate tests/golden/*.npz from the REFERENCE ITSELF, run in this container.
+"""Generate tests/golden/* from the REFERENCE ITSELF.
 
-Two sources (both need /root/reference, which exists only in the build container, never on the GPU box):
+Sources (all need a TinyChatEngine source tree, named by the environment variable TCE_REFERENCE_DIR):
 
 1. the reference's Python quantizer ``llm/tools/quantize_methods.py`` imported as-is -> packed INT4 formats
    (``quant_*.npz``): pins oracle/quant.py and tinychatengine_b200/formats.py byte-for-byte;
 2. the reference's C++ kernels compiled in place (``make -C oracle ref`` -> oracle/_ref/*.so, entered through
    oracle/ref_shim.cc) -> outputs of naive_mat_mul_int4 / int8_ref_matmul* / naive_mat_mul_int8 /
-   naive_mat_mul_fp16_int4 / the AVX W4A8 fast path (``kernels_*.npz``): pins oracle/tce_oracle.c.
+   naive_mat_mul_fp16_int4 / the AVX W4A8 fast path (``kernels_*.npz``): pins oracle/tce_oracle.c;
+3. the same builds on the seeded cases of tests/test_oracle_golden.py (``*_cases.npz``, ``int4_config1.npz``, ``norms.npz``) and
+   the layout of the reference's kernels/matmul.h (``matmul_h_layout.txt``);
+4. on a GPU, the reference's CUDA GEMV (oracle/_ref/libtce_ref_cuda.so, built beforehand) on the cases of
+   tests/test_gpu_w4a16.py::test_reference_cuda_kernel_on_this_gpu (``reference_cuda_gemv.npz``).
 
-Inputs are stored next to outputs, so the fixtures are self-contained.   Usage:  python tests/golden/make_golden.py
+Inputs are stored next to outputs, or regenerated from a seed by the test and fingerprinted, so the fixtures are self-contained.  Usage:
+
+    TCE_REFERENCE_DIR=<tree> python tests/golden/make_golden.py              # 1-3
+    TCE_REFERENCE_DIR=<tree> python tests/golden/make_golden.py recorded     # 3 only
+    python tests/golden/make_golden.py cuda OUT_DIR                          # 4, on a GPU: OUT_DIR/reference_cuda_gemv.npz
 """
 import os
 import sys
@@ -21,11 +29,20 @@ import numpy as np
 ROOT = Path(__file__).resolve().parents[2]
 sys.path.insert(0, str(ROOT))
 OUT = Path(__file__).resolve().parent
-REF_TOOLS = "/root/reference/llm/tools"
+TESTS = ROOT / "tests"
+
+
+def ref_tree() -> Path:
+    """The reference tree: its Python quantizer and headers are read directly, and capi.build() forwards it to oracle/Makefile as REF so
+    that oracle/_ref is built from the same tree."""
+    tree = os.environ.get("TCE_REFERENCE_DIR")
+    if not tree:
+        raise SystemExit("make_golden.py: set TCE_REFERENCE_DIR to a TinyChatEngine source tree")
+    return Path(tree)
 
 
 def ref_python_quantizer(w: np.ndarray, method: str):
-    sys.path.insert(0, REF_TOOLS)
+    sys.path.insert(0, str(ref_tree() / "llm" / "tools"))
     import quantize_methods as qm  # the reference module, unmodified
 
     oc, ic = w.shape
@@ -114,7 +131,7 @@ def main():
     np.savez_compressed(OUT / "kernels_generic.npz", **out)
 
     # the reference's AVX fast path (W4A8, g32): the timed CPU baseline; stored so the oracle/bench plumbing
-    # can be sanity-checked on a box without /root/reference
+    # can be sanity-checked without the reference tree
     X = capi.ref("avx")
     M, IC, OC = 1, 512, 64
     w = (rng.standard_normal((OC, IC)) * 0.02).astype(np.float32)
@@ -176,6 +193,7 @@ def main():
         samp[f"cfg{i}"] = np.array([c["top_k"], c["top_p"], c["temp"], c["repeat_penalty"], c["frequency_penalty"], c["presence_penalty"]], dtype=np.float64)
     np.savez_compressed(OUT / "sampling.npz", **samp)
     make_llama_model()
+    make_recorded_cases()
     print("golden fixtures written to", OUT)
 
 
@@ -202,5 +220,125 @@ def make_llama_model():
                         eps=np.float64(eps), tokens=tokens, logits=logits, weights_crc=np.uint32(crc))
 
 
+def _record(store, key, crc, **outputs):
+    store[f"{key}__crc"] = np.uint32(crc)
+    for name, a in outputs.items():
+        store[f"{key}__{name}"] = a
+
+
+def make_recorded_cases():
+    """The reference's outputs on the seeded cases of tests/test_oracle_golden.py (the test's own builders make the inputs) and the struct
+    layout of its kernels/matmul.h as printed by tests/test_host_header_abi.py's probe."""
+    import ctypes as C
+    import hashlib
+
+    from oracle import capi, llama_ref
+
+    sys.path.insert(0, str(TESTS))
+    import test_host_header_abi as ABI
+    import test_oracle_golden as T
+
+    capi.build(ref=True)
+    ref = ref_tree()
+    layout = ABI.probe(str(ref / "kernels" / "matmul.h"), ["-DQM_CUDA", "-I" + str(ref / "llm" / "half-2.2.0" / "include")])
+    (OUT / "matmul_h_layout.txt").write_text(layout + "\n")
+
+    rec = {}
+    for M in T.CONFIG1_M:
+        _, x, _, _, _, B, sc, crc = T.config1_case(M)
+        want = capi.ref_naive_mat_mul_int4(x.astype(np.float32), B, sc, 8.0, 128)
+        _record(rec, f"M{M}", crc, sha256=np.array(hashlib.sha256(want.tobytes()).hexdigest()), sample=want.ravel()[::T.CONFIG1_SAMPLE_STRIDE].copy())
+    np.savez_compressed(OUT / "int4_config1.npz", **rec)
+
+    rec = {}
+    for case in T.OPT_CASES:
+        E, H_, prefill, steps, _ = case
+        W, B, bo, hidden, par, crc = T.opt_attention_case(*case)
+        with tempfile.TemporaryDirectory() as d:
+            capi.write_opt_attention_params(d, W, B, bo, *par)
+            out, k, v = capi.ref_int8_opt_attention(d, hidden, E, H_, prefill, steps)
+        _record(rec, T.case_key(*case), crc, out=out, k=k, v=v)
+    np.savez_compressed(OUT / "opt_attention_cases.npz", **rec)
+
+    rec = {}
+    for case in T.LLAMA_ATTENTION_CASES:
+        E, H_, KVH, prefill, steps, _ = case
+        W, _, cosb, sinb, alpha, hidden, max_sq, crc = T.llama_attention_case(*case)
+        with tempfile.TemporaryDirectory() as d:
+            capi.write_llama_attention_params(d, W, cosb, sinb, alpha)
+            out, k, v = capi.ref_int4_llama_attention(d, hidden, E, H_, KVH, prefill, steps, max_sq)
+        _record(rec, T.case_key(*case), crc, out=out, k=k, v=v)
+    np.savez_compressed(OUT / "llama_attention_cases.npz", **rec)
+
+    rec = {}
+    X = capi.ref("avx")
+    for case in T.W4A8_CASES:
+        M, IC, OC, _ = case
+        A0, qs, d, crc = T.w4a8_case(*case)
+        A, Bq, S = (capi.aligned_empty(a.shape, a.dtype) for a in (A0, qs, d))  # the AVX kernels need aligned buffers
+        A[:], Bq[:], S[:] = A0, qs, d
+        Cx = capi.aligned_empty((M, OC), np.float32)
+        xi8 = capi.aligned_empty((M * IC,), np.int8)
+        xs = capi.aligned_empty((M * IC // 32,), np.float32)
+        X.ref_w4a8_avx(A.ctypes.data, Bq.ctypes.data, S.ctypes.data, Cx.ctypes.data, xi8.ctypes.data, xs.ctypes.data, M, IC, OC, 2)
+        _record(rec, T.case_key(*case), crc, C=np.array(Cx))
+    np.savez_compressed(OUT / "w4a8_avx_cases.npz", **rec)
+
+    rec = {}
+    for case in T.LLAMA_MODEL_CASES:
+        E, H_, KVH, L, F, V, prefill, steps, _ = case
+        model, tokens, cosb, sinb, crc = T.llama_model_case(*case)
+        with tempfile.TemporaryDirectory() as d:
+            llama_ref.write_llama_model_params(d, model, cosb, sinb, np.float32(1.0 / np.sqrt(E // H_)))
+            logits = llama_ref.ref_int4_llama_causal_lm(d, tokens, E, H_, KVH, L, F, V, prefill, steps, 640, 1e-6)
+        _record(rec, T.case_key(*case), crc, logits=logits)
+    np.savez_compressed(OUT / "llama_model_cases.npz", **rec)
+
+    rec = {}
+    Lm = C.CDLL(str(capi.REF_DIR / "libtce_ref_modules.so"))
+    vp = lambda a: a.ctypes.data_as(C.c_void_p)
+    for rows, dim, x, w, b, crc in T.norm_cases():
+        rms = np.zeros_like(x)
+        Lm.ref_llama_rmsnorm(vp(x), vp(w), vp(rms), rows, dim, C.c_float(1e-5))
+        x8 = (x * 20).astype(np.float32)
+        ln8 = np.zeros((rows, dim), np.int8)
+        Lm.ref_layernorm_q(vp(x8), vp(w), vp(b), vp(ln8), rows, dim)
+        _record(rec, T.case_key(rows, dim), crc, rmsnorm=rms, layernorm_q=ln8)
+    np.savez_compressed(OUT / "norms.npz", **rec)
+
+    rec = {}
+    for trial, logits, window, cfg, crc in T.sampling_trials():
+        ids, probs = capi.ref_sample_candidates(logits, window, **cfg)
+        _record(rec, f"trial{trial}", crc, ids=ids, probs=probs)
+    np.savez_compressed(OUT / "sampling_cases.npz", **rec)
+
+
+def make_reference_cuda_gemv(out_dir):
+    """On a GPU: the reference's gemv_kernel_g128 (oracle/_ref/libtce_ref_cuda.so) on the cases of test_reference_cuda_kernel_on_this_gpu."""
+    import torch
+
+    from oracle import capi
+
+    sys.path.insert(0, str(TESTS))
+    import test_gpu_w4a16 as T
+
+    rec = {}
+    for oc, ic in T.REFERENCE_CUDA_SHAPES:
+        x, w, z, s, crc = T.reference_cuda_case(oc, ic)
+        yr = torch.empty((1, oc), dtype=torch.float16, device=x.device)
+        torch.cuda.synchronize()
+        assert capi.ref_cuda().ref_cuda_gemv(x.data_ptr(), w.data_ptr(), z.data_ptr(), s.data_ptr(), yr.data_ptr(), 1, ic, oc) == 0
+        torch.cuda.synchronize()
+        _record(rec, f"{oc}x{ic}", crc, y=yr.cpu().numpy())
+    np.savez_compressed(Path(out_dir) / "reference_cuda_gemv.npz", **rec)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["recorded"]:
+        make_recorded_cases()
+    elif sys.argv[1:2] == ["cuda"] and len(sys.argv) == 3:
+        make_reference_cuda_gemv(sys.argv[2])
+    elif len(sys.argv) == 1:
+        main()
+    else:
+        raise SystemExit(__doc__)

@@ -10,7 +10,7 @@ import pytest
 from oracle import capi
 
 ROOT = Path(__file__).resolve().parents[1]
-pytestmark = pytest.mark.skipif(not capi.ref_available("avx"), reason="reference AVX build (oracle/_ref) not present")
+needs_reference_avx = pytest.mark.skipif(not capi.ref_available("avx"), reason="reference AVX build (oracle/_ref) not present")
 
 
 @pytest.fixture(scope="module")
@@ -21,6 +21,7 @@ def bench():
     return m
 
 
+@needs_reference_avx
 def test_w8a8_cpu_baseline_leg(bench):
     t0 = time.perf_counter()
     d = bench.cpu_baseline_w8a8(0.5)
@@ -31,6 +32,7 @@ def test_w8a8_cpu_baseline_leg(bench):
     assert abs(d["weight_GB_per_s"] * d["ms_per_layer_linears"] * 1e6 - (4 * 4096 * 4096 + 2 * 4096 * 11008)) < 1e3
 
 
+@needs_reference_avx
 def test_prefill_cpu_baseline_leg(bench):
     d = bench.cpu_baseline_prefill(2, model="tiny-gqa", m=32)
     json.dumps(d)
