@@ -228,21 +228,9 @@ int tce_w4a16_gemm(tce_ctx *ctx, const void *x, const void *w, const void *zeros
     if (IC < kW4Group || IC % kW4Group || OC < 1) return fail(TCE_ERR_INVALID, "tce_w4a16_gemm: bad shape M=%d IC=%d OC=%d", M, IC, OC);
     if (((uintptr_t)x | (uintptr_t)w | (uintptr_t)y) & 15) return fail(TCE_ERR_INVALID, "tce_w4a16_gemm: x, w, y must be 16-byte aligned");
     CK(cudaSetDevice(ctx->c.device), "cudaSetDevice");
-    const int mode = w4_gemm_mode();
-    if (mode == W4G_FUSED) {
-        CK(launch_gemm_w4_tc(&ctx->c, (const __half *)x, IC, (const uint32_t *)w, (const uint32_t *)zeros, (const __half *)scales, y, OC, M, OC, IC, 0), "tce_w4a16_gemm");
-        return TCE_OK;
-    }
-    if (mode == W4G_PAIR_FUSED) {
-        CK(launch_gemm_w4_pair(&ctx->c, (const __half *)x, IC, (const uint32_t *)w, (const uint32_t *)zeros, (const __half *)scales, y, OC, M, OC, IC, 0), "tce_w4a16_gemm");
-        return TCE_OK;
-    }
     CK(w4_scratch_reserve(&ctx->c, (size_t)OC * IC), "w16 scratch");
     CK(launch_w4_expand(&ctx->c, (const uint32_t *)w, (const uint32_t *)zeros, (const __half *)scales, ctx->c.w16_scratch, OC, IC), "w4_expand");
-    if (mode == W4G_PAIR || mode == W4G_PAIR_OVERLAP)  // a single call has no next linear to overlap with
-        CK(launch_gemm_f16_pair(&ctx->c, (const __half *)x, IC, ctx->c.w16_scratch, IC, (__half *)y, OC, M, OC, IC, 0), "tce_w4a16_gemm");
-    else
-        CK(launch_gemm_f16_tc(&ctx->c, (const __half *)x, IC, ctx->c.w16_scratch, IC, (__half *)y, OC, M, OC, IC), "tce_w4a16_gemm");
+    CK(launch_gemm_f16_pair(&ctx->c, (const __half *)x, IC, ctx->c.w16_scratch, IC, (__half *)y, OC, M, OC, IC, 0), "tce_w4a16_gemm");
     return TCE_OK;
 }
 

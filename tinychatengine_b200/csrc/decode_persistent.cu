@@ -23,7 +23,6 @@
 // 8-byte words, flag included) and every reader sums the P slots in rank order.
 // All waits are bounded: a protocol bug surfaces as a launch failure within seconds, not as a hung GPU.
 #include <stdio.h>
-#include <stdlib.h>
 
 #include "attention_impl.cuh"
 #include "persistent.h"
@@ -67,8 +66,8 @@ TCE_DEVINL uint2 ld_ll1(const uint2 *p, bool sys) {
 }
 // A failed poll waits this long before it asks L2 again: thousands of threads spinning without a pause fill the L2 request queues and
 // stretch every round trip (their own and the producers' stores) to ~0.5 us (profiles/README.md, run 11).
-__constant__ unsigned g_poll_ns = 100;  // TCE_PK_POLL_NS (set_poll_backoff)
-#define kPollBackoffNs g_poll_ns
+// Back-off 0 / 30 / 100 / 250 ns on one B200: 652 / 652 / 651 / 643 tok/s (profiles/README.md).
+constexpr unsigned kPollBackoffNs = 100;
 constexpr long long kSpinLimit = 20000000000LL;  // ~10 s: a peer rank may legitimately start its kernel later
 // spin until both words of the pair carry `tag`
 TCE_DEVINL uint4 wait_ll2(const uint2 *p, uint32_t tag, bool sys) {
@@ -148,26 +147,11 @@ TCE_DEVINL void mbar_wait_u32(uint32_t bar, uint32_t parity) {
 }
 TCE_DEVINL void mbar_arrive_u32(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); }
 
-// L2 prefetch of a TMA box / of a byte range: HBM -> L2 only, no shared-memory slot, no barrier
-TCE_DEVINL void tma_prefetch_2d_pred(const void *tmap, int x, int y, uint32_t pred) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %3, 0;\n\t@p cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];\n\t}" ::"l"(tmap), "r"(x), "r"(y),
-                 "r"(pred)
-                 : "memory");
-}
-TCE_DEVINL void tma_prefetch_3d_pred(const void *tmap, int x, int y, int z, uint32_t pred) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t@p cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];\n\t}" ::"l"(tmap), "r"(x),
-                 "r"(y), "r"(z), "r"(pred)
-                 : "memory");
-}
-TCE_DEVINL void bulk_prefetch_pred(const void *src, uint32_t bytes, uint32_t pred) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %2, 0;\n\t@p cp.async.bulk.prefetch.L2.global [%0], %1;\n\t}" ::"l"(src), "r"(bytes), "r"(pred) : "memory");
-}
 TCE_DEVINL int lds_volatile_i32(const int *p) {
     int v;
     asm volatile("ld.volatile.shared.s32 %0, [%1];" : "=r"(v) : "r"(smem_u32(p)) : "memory");
     return v;
 }
-TCE_DEVINL void sts_volatile_i32(int *p, int v) { asm volatile("st.volatile.shared.s32 [%0], %1;" ::"r"(smem_u32(p)), "r"(v) : "memory"); }
 
 TCE_DEVINL void stamp(const Args &a, int cta, int nphase, int p, int k) {  // one thread
     if (a.dbg) {
@@ -193,7 +177,6 @@ struct PSmem {
     float *rms;         // [kCW]
     float *rope;        // cos[128] | sin[128] of the token position
     uint64_t *full, *empty, *red_full, *red_empty;
-    int *issued;        // stages the loader has issued so far (read by the L2 prefetch warp)
     uint64_t *rx;       // pair staging: counts the bytes the partner has mirrored into this CTA for the current staging
     int *free_gen;      // pair staging: written by the partner: the number of phases it has finished (its buffers may be overwritten)
     uint32_t ring_u32, xs_u32, gx_u32, gsum_u32, full_u32, empty_u32, redfull_u32, redempty_u32;
@@ -225,8 +208,7 @@ TCE_DEVINL PSmem carve(uint8_t *raw, const Args &a) {
     s.red_full = s.empty + a.nst;
     s.red_empty = s.red_full + kRedBufs;
     s.rx = s.red_empty + kRedBufs;
-    s.issued = reinterpret_cast<int *>(s.rx + 1);
-    s.free_gen = s.issued + 1;
+    s.free_gen = reinterpret_cast<int *>(s.rx + 1);
     s.ring_u32 = smem_u32(s.ring);
     s.xs_u32 = smem_u32(s.xs);
     s.gx_u32 = smem_u32(s.gx);
@@ -295,41 +277,8 @@ TCE_DEVINL AttnSplit attn_split(int cta, int ncta, int KVH, int pos) {
 }
 
 // ------------------------------------------------------------------------------------------------------------ producer
-// The same walk over (tile, stage, box) serves two warps: the loader (PF = false) moves stages into the ring as slots free up; the
-// prefetcher (PF = true) runs `kPrefetchAhead` stages ahead of it and only asks L2 for the same boxes, so that the bytes in flight
-// towards HBM are not bounded by the ring (4 x 32 KiB per SM x ~3 us loaded HBM latency = ~40 GB/s per SM, the ceiling measured without
-// it, profiles/README.md) and a ring slot waits one L2 round trip instead of one DRAM round trip.
-constexpr int kPrefetchAhead = 10;
-struct ProdState {
-    Ring rs;
-    int count = 0;  // stages issued (loader) / prefetched (prefetcher) so far
-};
-template <bool PF>
-TCE_DEVINL void prod_throttle_or_slot(const PSmem &sm, ProdState &ps) {
-    if (PF) {
-        if (ps.count >= lds_volatile_i32(sm.issued) + kPrefetchAhead) {
-            const long long t0 = clock64();
-            while (ps.count >= lds_volatile_i32(sm.issued) + kPrefetchAhead) {
-                __nanosleep(64);
-                if (clock64() - t0 > kSpinLimit) __trap();
-            }
-        }
-    } else {
-        mbar_wait(&sm.empty[ps.rs.stage], ps.rs.phase ^ 1);
-    }
-}
-template <bool PF>
-TCE_DEVINL void prod_done(const PSmem &sm, ProdState &ps, uint32_t leader) {
-    ps.count++;
-    if (!PF) {
-        if (leader) sts_volatile_i32(sm.issued, ps.count);
-        __syncwarp();
-        ps.rs.advance(sm.nst);
-    }
-}
-
-template <bool PF>
-TCE_DEVINL void produce_gemv(const GemvOp &op, const CUtensorMap *m0, const uint8_t *meta, const PSmem &sm, ProdState &ps, int cta, int ncta, uint32_t leader,
+// The loader walks (tile, stage, box) in consumption order and moves every stage into the ring as soon as its slot is free.
+TCE_DEVINL void produce_gemv(const GemvOp &op, const CUtensorMap *m0, const uint8_t *meta, const PSmem &sm, Ring &rs, int cta, int ncta, uint32_t leader,
                              uint64_t policy) {
     int t0, t1;
     partition(op, cta, ncta, t0, t1);
@@ -337,22 +286,16 @@ TCE_DEVINL void produce_gemv(const GemvOp &op, const CUtensorMap *m0, const uint
     for (int tile = t0; tile < t1; tile++) {
         for (int s = 0; s < op.S; s++) {
             const BoxPlan &pl = op.plan[(ragged && s == op.S - 1) ? 1 : 0];
-            prod_throttle_or_slot<PF>(sm, ps);
-            uint64_t *bar = &sm.full[ps.rs.stage];
-            uint8_t *dst = sm.ring + (size_t)ps.rs.stage * kStageBytes;
-            if (!PF) mbar_arrive_expect_tx_pred(bar, (uint32_t)pl.bytes + kMetaBytes, leader);
+            mbar_wait(&sm.empty[rs.stage], rs.phase ^ 1);
+            uint64_t *bar = &sm.full[rs.stage];
+            uint8_t *dst = sm.ring + (size_t)rs.stage * kStageBytes;
+            mbar_arrive_expect_tx_pred(bar, (uint32_t)pl.bytes + kMetaBytes, leader);
 #pragma unroll 1
             for (int b = 0; b < pl.nbox; b++) {
                 const int xw = (kStageGroups * s + pl.b0[b]) * 16;  // first 32-bit word of the box within the row
                 uint8_t *d = dst + pl.off[b];
                 if (op.pair) {  // matrices of an op are kMapsPerMat maps apart
-                    if (PF && op.unit) {
-                        tma_prefetch_3d_pred(m0 + pl.map[b], 0, tile * 8, xw >> 4, leader);
-                        tma_prefetch_3d_pred(m0 + kMapsPerMat + pl.map[b], 0, tile * 8, xw >> 4, leader);
-                    } else if (PF) {
-                        tma_prefetch_2d_pred(m0 + pl.map[b], xw, tile * 8, leader);
-                        tma_prefetch_2d_pred(m0 + kMapsPerMat + pl.map[b], xw, tile * 8, leader);
-                    } else if (op.unit) {
+                    if (op.unit) {
                         tma_load_3d_pred(d, m0 + pl.map[b], 0, tile * 8, xw >> 4, bar, policy, leader);
                         tma_load_3d_pred(d + 8 * pl.bw[b] * 64, m0 + kMapsPerMat + pl.map[b], 0, tile * 8, xw >> 4, bar, policy, leader);
                     } else {
@@ -370,55 +313,41 @@ TCE_DEVINL void produce_gemv(const GemvOp &op, const CUtensorMap *m0, const uint
                             m = m0 + 2 * kMapsPerMat;
                         }
                     }
-                    if (PF && op.unit)
-                        tma_prefetch_3d_pred(m + pl.map[b], 0, row, xw >> 4, leader);
-                    else if (PF)
-                        tma_prefetch_2d_pred(m + pl.map[b], xw, row, leader);
-                    else if (op.unit)
+                    if (op.unit)
                         tma_load_3d_pred(d, m + pl.map[b], 0, row, xw >> 4, bar, policy, leader);
                     else
                         tma_load_2d_pred(d, m + pl.map[b], xw, row, bar, policy, leader);
                 }
             }
             const uint8_t *mrec = meta + ((size_t)tile * op.S + s) * kMetaBytes;
-            if (PF)
-                bulk_prefetch_pred(mrec, kMetaBytes, leader);
-            else
-                bulk_g2s_pred(dst + kMetaOff, mrec, kMetaBytes, bar, policy, leader);
-            prod_done<PF>(sm, ps, leader);
+            bulk_g2s_pred(dst + kMetaOff, mrec, kMetaBytes, bar, policy, leader);
+            __syncwarp();
+            rs.advance(sm.nst);
         }
     }
 }
 
-template <bool PF>
-TCE_DEVINL void produce_attn(const Args &a, const LayerDesc &L, const CUtensorMap *kvmap, const PSmem &sm, ProdState &ps, int cta, int ncta, int pos,
+TCE_DEVINL void produce_attn(const Args &a, const LayerDesc &L, const CUtensorMap *kvmap, const PSmem &sm, Ring &rs, int cta, int ncta, int pos,
                              uint32_t leader, uint64_t policy) {
     const AttnSplit sp = attn_split(cta, ncta, a.KVH, pos);
     for (int c = sp.ch0; c < sp.ch1; c++) {
-        prod_throttle_or_slot<PF>(sm, ps);
-        uint64_t *bar = &sm.full[ps.rs.stage];
-        uint8_t *dst = sm.ring + (size_t)ps.rs.stage * kStageBytes;
+        mbar_wait(&sm.empty[rs.stage], rs.phase ^ 1);
+        uint64_t *bar = &sm.full[rs.stage];
+        uint8_t *dst = sm.ring + (size_t)rs.stage * kStageBytes;
         const int krow = L.k_row0 + sp.kvh * a.max_ctx + c * kKvChunk, vrow = L.v_row0 + sp.kvh * a.max_ctx + c * kKvChunk;
-        if (PF) {
-            tma_prefetch_2d_pred(kvmap, 0, krow, leader);
-            tma_prefetch_2d_pred(kvmap, 64, krow, leader);
-            tma_prefetch_2d_pred(kvmap, 0, vrow, leader);
-            tma_prefetch_2d_pred(kvmap, 64, vrow, leader);
-        } else {
-            mbar_arrive_expect_tx_pred(bar, 2u * kHalfBytes, leader);
-            tma_load_2d_pred(dst, kvmap, 0, krow, bar, policy, leader);
-            tma_load_2d_pred(dst + 8192, kvmap, 64, krow, bar, policy, leader);
-            tma_load_2d_pred(dst + kHalfBytes, kvmap, 0, vrow, bar, policy, leader);
-            tma_load_2d_pred(dst + kHalfBytes + 8192, kvmap, 64, vrow, bar, policy, leader);
-        }
-        prod_done<PF>(sm, ps, leader);
+        mbar_arrive_expect_tx_pred(bar, 2u * kHalfBytes, leader);
+        tma_load_2d_pred(dst, kvmap, 0, krow, bar, policy, leader);
+        tma_load_2d_pred(dst + 8192, kvmap, 64, krow, bar, policy, leader);
+        tma_load_2d_pred(dst + kHalfBytes, kvmap, 0, vrow, bar, policy, leader);
+        tma_load_2d_pred(dst + kHalfBytes + 8192, kvmap, 64, vrow, bar, policy, leader);
+        __syncwarp();
+        rs.advance(sm.nst);
     }
 }
 
-// the producer role: PF = false on warp 0 (loader), PF = true on warp 2 (L2 prefetcher)
-template <bool PF>
+// the producer role (warp 0)
 TCE_DEVINL void producer_walk(const Args &a, const PSmem &sm, int cta, int ncta, int pos, int lane) {
-    ProdState ps;
+    Ring rs;
     const uint64_t policy = l2_policy_evict_first();
     const uint32_t leader = (lane == 0) ? 1u : 0u;
     const int Lyr = a.num_layers, nphase = 5 * Lyr + 1;
@@ -427,13 +356,13 @@ TCE_DEVINL void producer_walk(const Args &a, const PSmem &sm, int cta, int ncta,
     for (int p = 0; p < nphase; p++) {
         const int l = p / 5, k = p - 5 * l;
         if (l == Lyr) {
-            produce_gemv<PF>(a.op[OPI_LMHEAD], a.maps + (size_t)Lyr * 7 * kMapsPerMat, a.lm_meta, sm, ps, cta, ncta, leader, policy);
+            produce_gemv(a.op[OPI_LMHEAD], a.maps + (size_t)Lyr * 7 * kMapsPerMat, a.lm_meta, sm, rs, cta, ncta, leader, policy);
         } else if (k == 1) {
-            produce_attn<PF>(a, a.layers[l], kvmap, sm, ps, cta, ncta, pos, leader, policy);
+            produce_attn(a, a.layers[l], kvmap, sm, rs, cta, ncta, pos, leader, policy);
         } else {
             const int oi = (k == 0) ? OPI_QKV : (k - 1);       // k = 2,3,4 -> OPI_O, OPI_GATEUP, OPI_DOWN
             const int mi = (k == 0) ? 0 : (k == 2 ? 3 : (k == 3 ? 4 : 6));  // first tensor map of the op within the layer's seven
-            produce_gemv<PF>(a.op[oi], a.maps + ((size_t)l * 7 + mi) * kMapsPerMat, a.layers[l].meta[oi], sm, ps, cta, ncta, leader, policy);
+            produce_gemv(a.op[oi], a.maps + ((size_t)l * 7 + mi) * kMapsPerMat, a.layers[l].meta[oi], sm, rs, cta, ncta, leader, policy);
         }
     }
 }
@@ -1163,7 +1092,6 @@ __global__ void __launch_bounds__(kThreads, 1) decode_persistent_kernel(const __
             mbar_init(&sm.red_full[lane - 16], kCW);
             mbar_init(&sm.red_empty[lane - 16], 1);
         }
-        if (lane == 31) *sm.issued = 0;
         if (lane == 30) {
             mbar_init(sm.rx, 1);
             *sm.free_gen = 0;
@@ -1195,15 +1123,10 @@ __global__ void __launch_bounds__(kThreads, 1) decode_persistent_kernel(const __
     // and the 16 consumer warps grow to 112 (per scheduler: 32 + 4 x 112 <= 5 x 96 registers per lane)
     if (warp < kAuxWarps) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 32;" ::: "memory");
-        if (warp == 3) return;
+        if (warp >= 2) return;
         if (warp == 0) {
             // ================= loader: every byte this CTA needs from HBM, in consumption order =================
-            producer_walk<false>(a, sm, cta, ncta, pos, lane);
-            return;
-        }
-        if (warp == 2) {
-            // ================= L2 prefetcher: the same walk, kPrefetchAhead stages ahead =================
-            if (a.l2_prefetch) producer_walk<true>(a, sm, cta, ncta, pos, lane);
+            producer_walk(a, sm, cta, ncta, pos, lane);
             return;
         }
     if (warp == 1) {
@@ -1362,28 +1285,10 @@ __global__ void repack_meta_kernel(W4Seg s0, W4Seg s1, W4Seg s2, int nseg, int p
 BoxPlan make_box_plan(int n, int *widths, int *nwidths) {
     BoxPlan pl{};
     int w[kMaxBoxes], nb = 0;
-    // Dense boxes of up to 16 groups.  (Odd widths -- 9+9+7+7 -- make the weight LDS.128 conflict free, but rows of 576 / 448 bytes are
-    // not multiples of the 128-byte L2 line: measured 25 % SLOWER end to end, profiles/README.md; kept selectable for the record.)
-    const bool odd = getenv("TCE_PK_ODD_BOXES") != nullptr;
-    if (!odd) {
-        w[nb++] = n < 16 ? n : 16;
-        if (n > 16) w[nb++] = n - 16;
-    } else if (n <= 15 && (n & 1)) {
-        w[nb++] = n;
-    } else if (n <= 30) {
-        const int a = ((n / 2) & 1) ? n / 2 : n / 2 + 1;  // two odd parts
-        w[nb++] = a;
-        w[nb++] = n - a;
-    } else if (n == 31) {
-        w[nb++] = 15;
-        w[nb++] = 15;
-        w[nb++] = 1;
-    } else {  // 32
-        w[nb++] = 9;
-        w[nb++] = 9;
-        w[nb++] = 7;
-        w[nb++] = 7;
-    }
+    // Dense boxes of up to 16 groups: their rows are whole 128-byte L2 lines (odd widths, conflict-free but not line-aligned, measured
+    // 25 % slower end to end, profiles/README.md).
+    w[nb++] = n < 16 ? n : 16;
+    if (n > 16) w[nb++] = n - 16;
     int g0 = 0, off = 0;
     for (int i = 0; i < nb; i++) {
         pl.b0[i] = g0;
@@ -1414,6 +1319,7 @@ int attn_nsplit_max(int ncta, int KVH, int max_ctx) {
     return NS < nch ? NS : nch;
 }
 
+// everything next to the ring; the 16 bytes after the barriers hold the rx barrier and free_gen (padded)
 static size_t fixed_bytes(int xs_bytes, int max_ng, int E) {
     return (size_t)xs_bytes + (size_t)E * 4 + (size_t)max_ng * 12 + (size_t)kRedBufs * kCW * 16 * 4 + 32 * 4 + 256 * 4 + (size_t)(2 * kMaxStages + 2 * kRedBufs) * 8 + 16 + 1024;
 }
@@ -1478,8 +1384,6 @@ bool pair_supported(Ctx *ctx, const Args &a) {
     }
     return nclusters * 2 >= ctx->num_sms;
 }
-
-cudaError_t set_poll_backoff(unsigned ns) { return cudaMemcpyToSymbol(g_poll_ns, &ns, sizeof(ns)); }
 
 cudaError_t launch(Ctx *ctx, const Args &a, cudaStream_t stream) {
     const size_t smem = smem_bytes(a);

@@ -1,10 +1,10 @@
-// gemm_tc.cuh -- the large-M GEMM of the path on the 5th-generation tensor cores:  C[M][N] = A[M][K] * B[N][K]^T with both operands
+// gemm_tc.cuh -- the large-M int8 GEMM of the path on the 5th-generation tensor cores:  C[M][N] = A[M][K] * B[N][K]^T with both operands
 // K-major, which is the natural layout of the activations ([tokens][IC]) and of the weights ([OC][IC]) on this path.
 //
-//   * operands reach shared memory by 2-D TMA (128-byte swizzle, one 128-byte swizzle atom of K per stage row: 64 fp16 or 128 int8),
-//   * one elected thread issues tcgen05.mma (cta_group::1, M = 128, N = BLOCK_N, K = 32 bytes per instruction) straight from the
+//   * operands reach shared memory by 2-D TMA (128-byte swizzle, one 128-byte swizzle atom of K = 128 int8 per stage row),
+//   * one elected thread issues tcgen05.mma.kind::i8 (cta_group::1, M = 128, N = BLOCK_N, K = 32 per instruction) straight from the
 //     swizzled tiles through shared-memory matrix descriptors,
-//   * the fp32 / int32 accumulator lives in TMEM, double buffered (2 x BLOCK_N columns), so the epilogue of tile i overlaps the
+//   * the int32 accumulator lives in TMEM, double buffered (2 x BLOCK_N columns), so the epilogue of tile i overlaps the
 //     main loop of tile i+1,
 //   * four epilogue warps read their 32-lane quarter of TMEM with tcgen05.ld and apply the op's epilogue in registers.
 // Persistent: one CTA per SM walks tiles m-fastest so that concurrently running CTAs share the same B (weight) tile in L2.
@@ -28,7 +28,7 @@ struct GemmArgs {
     alignas(64) CUtensorMap tmA;  // [M][K] box {128 B, 128 rows}
     alignas(64) CUtensorMap tmB;  // [N][K] box {128 B, BLOCK_N rows}
     int M, N;
-    int k_blocks;                 // K * sizeof(element) / 128
+    int k_blocks;                 // K / 128
     int m_blocks, n_blocks;
     // epilogue
     void *C;
@@ -52,17 +52,10 @@ TCE_DEVINL void tmem_dealloc(uint32_t taddr, uint32_t ncols) {  // whole warp
 TCE_DEVINL void umma_commit(uint64_t *bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-template <bool I8>
-TCE_DEVINL void umma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    if constexpr (I8) {
-        asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d), "l"(adesc),
-                     "l"(bdesc), "r"(idesc), "r"(accumulate)
-                     : "memory");
-    } else {
-        asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d), "l"(adesc),
-                     "l"(bdesc), "r"(idesc), "r"(accumulate)
-                     : "memory");
-    }
+TCE_DEVINL void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d), "l"(adesc),
+                 "l"(bdesc), "r"(idesc), "r"(accumulate)
+                 : "memory");
 }
 // 32 lanes x 32 consecutive 32-bit columns: thread t of the warp receives row (lane quarter base + t), columns c..c+31
 TCE_DEVINL void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
@@ -92,11 +85,11 @@ TCE_DEVINL uint64_t make_sw128_desc(uint32_t smem_addr) {
     return ((uint64_t)hi << 32) | lo;
 }
 
-// instruction descriptor: c_format [4,6) (1 = F32, 2 = S32), a_format [7,10), b_format [10,13) (F16 = 0; INT8 signed = 1),
+// instruction descriptor: c_format [4,6) (2 = S32), a_format [7,10), b_format [10,13) (INT8 signed = 1),
 // a/b major bits 15/16 = 0 (K-major), N >> 3 in [17,23), M >> 4 in [24,29)
-template <int BLOCK_N, bool I8>
-constexpr uint32_t make_idesc() {
-    return (I8 ? (2u << 4) | (1u << 7) | (1u << 10) : (1u << 4)) | ((uint32_t)(BLOCK_N >> 3) << 17) | ((uint32_t)(kBlockM >> 4) << 24);
+template <int BLOCK_N>
+constexpr uint32_t make_idesc_i8() {
+    return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BLOCK_N >> 3) << 17) | ((uint32_t)(kBlockM >> 4) << 24);
 }
 
 template <int BLOCK_N, int STAGES>
@@ -105,7 +98,7 @@ constexpr size_t smem_bytes() {
 }
 
 // Epi::apply(args, row, col0, ncols_valid, v[32]) consumes 32 consecutive accumulator columns of one output row.
-template <int BLOCK_N, int STAGES, bool I8, class Epi>
+template <int BLOCK_N, int STAGES, class Epi>
 __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_constant__ GemmArgs a) {
     static_assert(BLOCK_N == 128 || BLOCK_N == 192 || BLOCK_N == 256, "BLOCK_N");
     constexpr int kBBytes = BLOCK_N * kAtomBytes;
@@ -149,7 +142,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
                 for (int kb = 0; kb < a.k_blocks; kb++) {
                     mbar_wait(&empty_bar[s], ph ^ 1u);
                     mbar_arrive_expect_tx(&full_bar[s], kABytes + kBBytes);
-                    const int kx = kb * (I8 ? kAtomBytes : kAtomBytes / 2);  // element coordinate along K
+                    const int kx = kb * kAtomBytes;  // element coordinate along K
                     tma_load_2d(sA + (size_t)s * kABytes, &a.tmA, kx, mb * kBlockM, &full_bar[s]);
                     tma_load_2d(sB + (size_t)s * kBBytes, &a.tmB, kx, nb * BLOCK_N, &full_bar[s]);
                     if (++s == STAGES) {
@@ -163,7 +156,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
     } else if (warp == 1) {
         // ------------------------------------------------------------------------------- MMA issuer
         if (lane == 0) {
-            constexpr uint32_t idesc = make_idesc<BLOCK_N, I8>();
+            constexpr uint32_t idesc = make_idesc_i8<BLOCK_N>();
             int s = 0;
             uint32_t ph = 0;
             int it = 0;
@@ -180,7 +173,7 @@ __global__ void __launch_bounds__(kThreads, 1) gemm_tc_kernel(const __grid_const
                     const uint64_t bdesc = make_sw128_desc(smem_u32(sB + (size_t)s * kBBytes));
 #pragma unroll
                     for (int k = 0; k < kAtomBytes / 32; k++)  // 32 bytes of K per instruction; +2 in the (>>4) address field
-                        umma<I8>(tmem_d, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) != 0 ? 1u : 0u);
+                        umma_i8(tmem_d, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) != 0 ? 1u : 0u);
                     umma_commit(&empty_bar[s]);  // smem slot reusable once these MMAs have read it
                     if (++s == STAGES) {
                         s = 0;

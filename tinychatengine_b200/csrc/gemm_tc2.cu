@@ -1,20 +1,15 @@
-// gemm_tc2.cu -- the prefill GEMM on CTA pairs:  C[M][N] = X[M][K] (fp16) * W[N][K]^T, tcgen05.mma.cta_group::2.
+// gemm_tc2.cu -- the W4A16 prefill GEMM (MatmulOperator::gemm_forward_cuda, declared-but-undefined in the reference,
+// kernels/matmul.h:142-145): the QM_CUDA int4 weights are expanded to fp16 ((q - z) * s, one rounding) by a bandwidth-bound pass, then
+// C[M][N] = X[M][K] (fp16) * W[N][K]^T runs on CTA pairs with tcgen05.mma.cta_group::2 and fp32 accumulation in TMEM.  Expanding once
+// per call instead of once per M tile keeps the CUDA-core dequant work at OC*IC instead of OC*IC*ceil(M/256).
 //
 // Two CTAs of a cluster (one TPC) own one 256 x 256 output tile.  Each CTA stages ITS 128 activation rows and ITS 128 weight rows of
 // every 64-k block; one thread of the leader CTA issues M = 256 MMAs that read both CTAs' shared memory, so per CTA and k-block the
 // tensor core pulls 32 KiB of operands for 128 x 256 x 64 MACs -- half of what a single-CTA 128 x 256 tile needs, which is what bounds
-// the single-CTA kernel (gemm_tc.cuh): there the operand reads + TMA writes (+ dequant traffic when fused) exceed the 128 B/clk of one SM's
-// shared memory long before the tensor pipe is busy (profiles/README.md, round 2).
-//
-// FUSED = false: W is fp16 (the expanded scratch): both operands arrive by TMA (cta_group::2 flavour: completion bytes are counted on the
-//                leader's mbarrier).
-// FUSED = true:  W is the packed QM_CUDA int4 matrix: each CTA's TMA brings 128 rows x 32 bytes of nibbles per k-block, four dequant warps turn
-//                them into the fp16 K-major SWIZZLE_128B operand tile ((q - z) * s, exact subtraction, one rounding), fence.proxy.async, and
-//                arrive on the LEADER's barrier (remote arrive from the peer).  Nothing but the nibbles crosses HBM for the weights.
+// a single-CTA kernel: there the operand reads + TMA writes exceed the 128 B/clk of one SM's shared memory long before the tensor pipe
+// is busy (profiles/README.md, round 2).  Both operands arrive by TMA (cta_group::2 flavour: completion bytes are counted on the
+// leader's mbarrier).
 // Epilogue: every CTA reads its own 128 accumulator rows from its own TMEM (double-buffered accumulators), fp16 store or fp32 accumulate.
-#include <cstdlib>
-#include <string>
-
 #include "gemm_tc.cuh"
 #include "kernels.h"
 
@@ -26,36 +21,22 @@ using namespace tc;
 constexpr int kPairN = 256;                 // output columns per tile (each CTA stages half of the weight rows)
 constexpr int kHalfN = 128;
 constexpr int kBHalfBytes = kHalfN * 128;   // 16 KiB fp16 operand tile per CTA and k-block
-constexpr int kRawHalf = kHalfN * 32;       // 4 KiB of packed nibbles
-constexpr int kDq = 4;                      // dequant warps per k-block and CTA (FUSED): one thread per weight row
-constexpr int kDqGroups = 2;                // groups of kDq warps working on alternate k-blocks (hides the per-block barrier / fence latencies)
+constexpr int kStages = 6;                  // ring of activation tiles + this CTA's fp16 weight tile in the same slot
+constexpr int kSlotBytes = kABytes + kBHalfBytes;
+constexpr int kPairThreads = 32 * 6;
+constexpr size_t kPairSmem = 1024 + (size_t)kStages * kSlotBytes;
 constexpr uint32_t kPeerMask = 0xFEFFFFFFu; // clears the CTA-rank bit of a shared::cluster address: "the same location in CTA 0"
 constexpr uint64_t kEvictNormal = 0x1000000000000000ull;
 
-template <bool FUSED>
-struct Cfg {
-    static constexpr int kAStages = 6;               // ring of activation tiles (not FUSED: + this CTA's fp16 weight tile in the same slot)
-    static constexpr int kOpStages = FUSED ? 4 : 0;  // ring of dequantised operand tiles
-    static constexpr int kRawStages = FUSED ? 12 : 0;  // ring of packed weight tiles: its own, deeper ring -- 4 KiB per k-block buys the look-ahead
-                                                       // that hides the load latency in front of the dequant warps (a shared 5-slot ring left the
-                                                       // tensor pipe at 42 %: a slot was only re-requested after its MMA had retired)
-    static constexpr int kSlotBytes = kABytes + (FUSED ? 0 : kBHalfBytes);
-    static constexpr int kThreads = 32 * (6 + (FUSED ? kDq * kDqGroups + 1 : 0));  // FUSED: + one warp that loads the packed tiles
-    static constexpr size_t kSmem = 1024 + (size_t)kAStages * kSlotBytes + (size_t)kOpStages * kBHalfBytes + (size_t)kRawStages * kRawHalf;
-};
-
 struct PairArgs {
     alignas(64) CUtensorMap tmA;  // fp16 [M][K], box {64, 128}, SWIZZLE_128B
-    alignas(64) CUtensorMap tmB;  // FUSED: uint32 [N][K/8], box {8, 128}, no swizzle; else fp16 [N][K], box {64, 128}, SWIZZLE_128B
-    const __half *scales;
-    const uint32_t *zeros;
-    int sf_w, zeros_w;
+    alignas(64) CUtensorMap tmB;  // fp16 [N][K], box {64, pn / 2}, SWIZZLE_128B
     int M, N, k_blocks, m_blocks, n_blocks;  // blocks of 256
     void *C;
     long long ldc;
     int add_f32;
     int pn;      // output columns per tile of the fp16-weight kernel: 256, or 128 where 256-wide tiles quantise badly onto the 74 clusters (N = 5120:
-                 // 160 tiles = 2.16 waves); each CTA stages pn / 2 weight rows.  The fused and SiLU variants use 256.
+                 // 160 tiles = 2.16 waves); each CTA stages pn / 2 weight rows.  The SiLU variant uses 256.
     int silu_F;  // > 0: W = [gate (F rows); up (F rows)], the pair's two halves are the SAME 128 channels of gate (CTA 0) and up (CTA 1), and the
                  // epilogue writes act[M][F] = SiLU(gate) * up (SiLuMul_half, llm/src/nn_modules/cuda/Int4llamaDecoderLayer.cu:12-30; fp32 math)
 };
@@ -83,8 +64,8 @@ TCE_DEVINL void cluster_sync_all() {
 TCE_DEVINL void mbar_arrive_cluster(uint64_t *bar, uint32_t rank) {
     uint32_t remote;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(smem_u32(bar)), "r"(rank));
-    // default semantics (release at CTA scope), as for a local arrive: the operand tile was already published to the async proxy by
-    // fence.proxy.async; a cluster-scope release costs MEMBAR.ALL.GPU + ERRBAR per arrive and halved the kernel (profiles/README.md)
+    // default semantics (release at CTA scope), as for a local arrive: the caller's tcgen05.fence::before_thread_sync orders its TMEM reads;
+    // a cluster-scope release costs MEMBAR.ALL.GPU + ERRBAR per arrive (profiles/README.md)
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(remote) : "memory");
 }
 // wait on a barrier whose arrivals come from both CTAs (plain try_wait: an acquire.cluster wait invalidates L1 on every poll)
@@ -125,37 +106,14 @@ TCE_DEVINL void umma_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint3
                  : "memory");
 }
 
-TCE_DEVINL uint32_t lop3_and_or2(uint32_t a, uint32_t b, uint32_t c) {
-    uint32_t r;
-    asm("lop3.b32 %0, %1, %2, %3, 0xEA;" : "=r"(r) : "r"(a), "r"(b), "r"(c));
-    return r;
-}
-TCE_DEVINL uint4 dequant_word2(uint32_t w, uint32_t zmagic, __half2 s2) {  // 8 nibbles -> 8 fp16 (q - z) * s in k order
-    constexpr uint32_t Mk = 0x000F000Fu, MG = 0x64006400u;
-    const __half2 zm = *reinterpret_cast<const __half2 *>(&zmagic);
-    uint32_t q[4] = {lop3_and_or2(w, Mk, MG), lop3_and_or2(w >> 4, Mk, MG), lop3_and_or2(w >> 8, Mk, MG), lop3_and_or2(w >> 12, Mk, MG)};
-    uint32_t p[4];
-#pragma unroll
-    for (int i = 0; i < 4; i++) {
-        const __half2 v = __hmul2(__hsub2(*reinterpret_cast<const __half2 *>(&q[i]), zm), s2);
-        p[i] = *reinterpret_cast<const uint32_t *>(&v);
-    }
-    return make_uint4(__byte_perm(p[0], p[1], 0x5410), __byte_perm(p[2], p[3], 0x5410), __byte_perm(p[0], p[1], 0x7632), __byte_perm(p[2], p[3], 0x7632));
-}
-
-template <bool FUSED>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads, 1) gemm_pair_kernel(const __grid_constant__ PairArgs a) {
-    using C = Cfg<FUSED>;
-    constexpr int AS = C::kAStages, OS = FUSED ? C::kOpStages : 1, RS = FUSED ? C::kRawStages : 1;
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kPairThreads, 1) gemm_pair_kernel(const __grid_constant__ PairArgs a) {
+    constexpr int AS = kStages;
     extern __shared__ uint8_t smem_raw[];
     // barriers live at identical offsets in both CTAs (multicast commits and remote arrives address "the same barrier in the other CTA")
-    __shared__ __align__(8) uint64_t a_full[AS], a_empty[AS], raw_full[RS], raw_empty[RS], op_full[OS], op_empty[OS], tfull_bar[2], tempty_bar[2];
+    __shared__ __align__(8) uint64_t a_full[AS], a_empty[AS], tfull_bar[2], tempty_bar[2];
     __shared__ uint32_t tmem_base_s;
     const uint32_t raw = smem_u32(smem_raw);
-    uint8_t *base = smem_raw + (((raw + 1023u) & ~1023u) - raw);
-    uint8_t *sSlot = base;                                    // [AS][A 16 KiB (| B half fp16 16 KiB when not FUSED)]
-    uint8_t *sOp = base + (size_t)AS * C::kSlotBytes;         // FUSED: [OS][16 KiB] dequantised operand tiles
-    uint8_t *sRaw = sOp + (size_t)(FUSED ? OS : 0) * kBHalfBytes;  // FUSED: [RS][4 KiB] packed tiles
+    uint8_t *sSlot = smem_raw + (((raw + 1023u) & ~1023u) - raw);  // [AS][A 16 KiB | B half fp16 16 KiB]
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_rank();
     const bool leader = rank == 0;
@@ -166,14 +124,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
         for (int s = 0; s < AS; s++) {
             mbar_init(&a_full[s], 1);                          // leader: its own expect_tx arrival; bytes from both CTAs
             mbar_init(&a_empty[s], 1);                         // multicast MMA commit
-        }
-        for (int s = 0; s < RS; s++) {
-            mbar_init(&raw_full[s], 1);                        // FUSED: this CTA's packed tile (local TMA)
-            mbar_init(&raw_empty[s], kDq);                     // the dequant warps of the group that owns the k-block
-        }
-        for (int s = 0; s < OS; s++) {
-            mbar_init(&op_full[s], 2 * kDq);                   // leader: dequant warps of both CTAs
-            mbar_init(&op_empty[s], 1);                        // multicast MMA commit
         }
         for (int s = 0; s < 2; s++) {
             mbar_init(&tfull_bar[s], 1);                       // multicast MMA commit
@@ -198,19 +148,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
             for (int t = cl; t < tiles_total; t += ncl) {
                 const int mb = t % a.m_blocks, nb = t / a.m_blocks;
                 const int row0 = mb * 256 + (int)rank * kBlockM;
-                const int pn = FUSED ? kPairN : a.pn, hn = pn >> 1;
+                const int pn = a.pn, hn = pn >> 1;
                 const int wrow0 = a.silu_F > 0 ? nb * kHalfN + (int)rank * a.silu_F : nb * pn + (int)rank * hn;
                 for (int kb = 0; kb < a.k_blocks; kb++) {
                     mbar_wait(&a_empty[s], ph ^ 1u);
-                    uint8_t *dst = sSlot + (size_t)s * C::kSlotBytes;
-                    if (FUSED) {
-                        if (leader) mbar_arrive_expect_tx(&a_full[s], 2 * kABytes);
-                        tma_load_2d_pair(dst, &a.tmA, kb * 64, row0, &a_full[s]);
-                    } else {
-                        if (leader) mbar_arrive_expect_tx(&a_full[s], 2 * (kABytes + hn * 128));
-                        tma_load_2d_pair(dst, &a.tmA, kb * 64, row0, &a_full[s]);
-                        tma_load_2d_pair(dst + kABytes, &a.tmB, kb * 64, wrow0, &a_full[s]);
-                    }
+                    uint8_t *dst = sSlot + (size_t)s * kSlotBytes;
+                    if (leader) mbar_arrive_expect_tx(&a_full[s], 2 * (kABytes + hn * 128));
+                    tma_load_2d_pair(dst, &a.tmA, kb * 64, row0, &a_full[s]);
+                    tma_load_2d_pair(dst + kABytes, &a.tmB, kb * 64, wrow0, &a_full[s]);
                     if (++s == AS) {
                         s = 0;
                         ph ^= 1u;
@@ -222,9 +167,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
     } else if (warp == 1) {
         // ------------------------------------------------------------------------------- MMA issuer (leader CTA only)
         if (leader && lane == 0) {
-            const uint32_t idesc = (1u << 4) | ((uint32_t)((FUSED ? kPairN : a.pn) >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);  // F32 acc, f16 x f16, K-major, N, M 256
-            int s = 0, os = 0, it = 0;
-            uint32_t ph = 0, oph = 0;
+            const uint32_t idesc = (1u << 4) | ((uint32_t)(a.pn >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);  // F32 acc, f16 x f16, K-major, N, M 256
+            int s = 0, it = 0;
+            uint32_t ph = 0;
             for (int t = cl; t < tiles_total; t += ncl, it++) {
                 const int acc = it & 1;
                 const uint32_t acc_ph = (uint32_t)(it >> 1) & 1u;
@@ -233,28 +178,22 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
                 const uint32_t tmem_d = tmem_base + (uint32_t)(acc * kPairN);
                 for (int kb = 0; kb < a.k_blocks; kb++) {
                     mbar_wait(&a_full[s], ph);
-                    if (FUSED) mbar_wait_cl(&op_full[os], oph);
                     tc_fence_after();
-                    const uint64_t adesc = make_sw128_desc(smem_u32(sSlot + (size_t)s * C::kSlotBytes));
-                    const uint64_t bdesc = make_sw128_desc(FUSED ? smem_u32(sOp + (size_t)os * kBHalfBytes) : smem_u32(sSlot + (size_t)s * C::kSlotBytes + kABytes));
+                    const uint64_t adesc = make_sw128_desc(smem_u32(sSlot + (size_t)s * kSlotBytes));
+                    const uint64_t bdesc = make_sw128_desc(smem_u32(sSlot + (size_t)s * kSlotBytes + kABytes));
 #pragma unroll
                     for (int k = 0; k < 4; k++) umma_pair(tmem_d, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (kb | k) != 0 ? 1u : 0u);
                     umma_commit_pair(&a_empty[s]);
-                    if (FUSED) umma_commit_pair(&op_empty[os]);
                     if (++s == AS) {
                         s = 0;
                         ph ^= 1u;
-                    }
-                    if (FUSED && ++os == OS) {
-                        os = 0;
-                        oph ^= 1u;
                     }
                 }
                 umma_commit_pair(&tfull_bar[acc]);
             }
         }
         __syncwarp();
-    } else if (warp < 6) {
+    } else {
         // ------------------------------------------------------------------------------- epilogue (both CTAs, own accumulator rows)
         const int q = warp & 3;
         int it = 0;
@@ -291,7 +230,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
                 mbar_arrive_cluster(&tempty_bar[acc], 0);
                 continue;
             }
-            const int pn = FUSED ? kPairN : a.pn;
+            const int pn = a.pn;
 #pragma unroll 1
             for (int c = 0; c < pn / 32; c++) {
                 uint32_t v[32];
@@ -340,77 +279,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
             tc_fence_before();
             mbar_arrive_cluster(&tempty_bar[acc], 0);  // the leader's MMA thread may overwrite this accumulator (in both CTAs)
         }
-    } else if (FUSED && warp == 6 + kDq * kDqGroups) {
-        // ------------------------------------------------------------------------------- packed-weight producer (both CTAs, local barriers)
-        if (lane == 0) {
-            int s = 0;
-            uint32_t ph = 0;
-            for (int t = cl; t < tiles_total; t += ncl) {
-                const int nb = t / a.m_blocks;
-                const int wrow0 = nb * kPairN + (int)rank * kHalfN;
-                for (int kb = 0; kb < a.k_blocks; kb++) {
-                    mbar_wait(&raw_empty[s], ph ^ 1u);
-                    mbar_arrive_expect_tx(&raw_full[s], kRawHalf);
-                    tma_load_2d(sRaw + (size_t)s * kRawHalf, &a.tmB, kb * 8, wrow0, &raw_full[s]);
-                    if (++s == RS) {
-                        s = 0;
-                        ph ^= 1u;
-                    }
-                }
-            }
-        }
-        __syncwarp();
-    } else if (FUSED) {
-        // ------------------------------------------------------------------------------- dequant warps: thread r owns weight row r of this CTA's half;
-        // group `grp` takes the k-blocks kb = grp (mod kDqGroups).  K % 128 == 0 makes k_blocks even, so a group sees the same half of every
-        // 128-k scale group in every tile.
-        const int dt = threadIdx.x - 32 * 6;
-        const int r = dt & (kHalfN - 1), grp = dt >> 7;
-        const uint32_t row_off = (uint32_t)(r >> 3) * 1024u + (uint32_t)(r & 7) * 128u;
-        const uint32_t sw = (uint32_t)(r & 7);
-        long long kbase = 0;  // k-blocks of the tiles processed so far: ring slot = (kbase + kb) % depth
-        for (int t = cl; t < tiles_total; t += ncl) {
-            const int nb = t / a.m_blocks;
-            const int grow = nb * kPairN + (int)rank * kHalfN + r;
-            const bool live = grow < a.N;
-            const __half *srow = a.scales + (size_t)(live ? grow : 0) * a.sf_w;
-            const uint32_t *zrow = a.zeros + (size_t)(live ? grow : 0) * a.zeros_w;
-            // scale / zero point of a 128-k group are requested one group before they are used (an L2 round trip on this critical path otherwise)
-            const int ngroups = a.k_blocks >> 1;
-            uint32_t zword = 0u, zword_nxt = live ? zrow[0] : 0u;
-            __half s_nxt = live ? srow[0] : __float2half(0.f);
-            for (int kb = grp; kb < a.k_blocks; kb += kDqGroups) {
-                const int g = kb >> 1;  // kDqGroups == 2: every iteration of a group is a new scale group
-                if ((g & 7) == 0) {
-                    zword = zword_nxt;
-                    if (live && g + 8 < ngroups) zword_nxt = zrow[(g >> 3) + 1];
-                }
-                const uint32_t z = (zword >> (4 * (g & 7))) & 0xFu;
-                const uint32_t zmagic = 0x64006400u | z | (z << 16);
-                const __half2 s2 = __half2half2(s_nxt);
-                if (live && g + 1 < ngroups) s_nxt = srow[g + 1];
-                const long long kk = kbase + kb;
-                const int s = (int)(kk % RS), os = (int)(kk % OS);
-                const uint32_t ph = (uint32_t)((kk / RS) & 1), oph = (uint32_t)((kk / OS) & 1);
-                mbar_wait(&raw_full[s], ph);
-                const uint8_t *src = sRaw + (size_t)s * kRawHalf + (size_t)r * 32;
-                const uint4 w0 = *reinterpret_cast<const uint4 *>(src), w1 = *reinterpret_cast<const uint4 *>(src + 16);
-                __syncwarp();
-                if (lane == 0) mbar_arrive(&raw_empty[s]);  // the packed tile is in registers
-                const uint32_t ww[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-                uint4 o[8];
-#pragma unroll
-                for (int c = 0; c < 8; c++) o[c] = dequant_word2(ww[c], zmagic, s2);
-                mbar_wait(&op_empty[os], oph ^ 1u);
-                uint8_t *dst = sOp + (size_t)os * kBHalfBytes + row_off;
-#pragma unroll
-                for (int c = 0; c < 8; c++) *reinterpret_cast<uint4 *>(dst + (((uint32_t)c ^ sw) << 4)) = o[c];
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cluster(&op_full[os], 0);
-            }
-            kbase += a.k_blocks;
-        }
     }
     tc_fence_before();
     cluster_sync_all();  // both CTAs are done with TMEM and with each other's shared memory
@@ -418,6 +286,30 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(Cfg<FUSED>::kThreads
         tc_fence_after();
         tmem_dealloc_pair(tmem_base, 512);
     }
+}
+
+// W4 -> fp16 expansion: // one thread per 32-bit word (8 sequential nibbles, weights 8c..8c+7 of row o) -> one 16-byte store
+__global__ void w4_expand_kernel(const uint32_t *__restrict__ w, const uint32_t *__restrict__ zeros, const __half *__restrict__ scales, __half *__restrict__ out,
+                                 int OC, int words_per_row, int zeros_w, int sf_w) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (long long)OC * words_per_row) return;
+    const int o = (int)(idx / words_per_row), c = (int)(idx % words_per_row);
+    const int g = c >> 4;  // 16 words = 128 weights per group
+    const uint32_t z = (zeros[(size_t)o * zeros_w + (g >> 3)] >> (4 * (g & 7))) & 0xFu;
+    const __half s = scales[(size_t)o * sf_w + g];
+    const __half2 s2 = __half2half2(s);
+    const uint32_t zmagic = 0x64006400u | z | (z << 16);  // (1024 + z) in both halves
+    const uint32_t word = w[idx];
+    uint32_t r[4];
+#pragma unroll
+    for (int p = 0; p < 4; p++) {
+        const uint32_t x = word >> (8 * p);
+        const uint32_t qmagic = 0x64006400u | (x & 0xFu) | ((x & 0xF0u) << 12);  // (1024 + q) for weights 2p, 2p+1
+        const __half2 d = __hsub2(*reinterpret_cast<const __half2 *>(&qmagic), *reinterpret_cast<const __half2 *>(&zmagic));  // exact
+        const __half2 m = __hmul2(d, s2);                                                                                     // one rounding
+        r[p] = *reinterpret_cast<const uint32_t *>(&m);
+    }
+    reinterpret_cast<uint4 *>(out)[idx] = make_uint4(r[0], r[1], r[2], r[3]);
 }
 
 typedef CUresult (*EncodeFn2)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
@@ -441,38 +333,40 @@ bool encode_f16(CUtensorMap *out, const void *base, long long rows, long long K,
                       CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <bool FUSED>
 cudaError_t launch_pair(Ctx *ctx, PairArgs &a) {
-    using C = Cfg<FUSED>;
-    auto kern = gemm_pair_kernel<FUSED>;
     static DeviceOnce attr_once;
     if (attr_once.pending(ctx->device)) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::kSmem);
+        cudaError_t e = cudaFuncSetAttribute(gemm_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPairSmem);
         if (e != cudaSuccess) return e;
         attr_once.done(ctx->device);
     }
     const int tiles = a.m_blocks * a.n_blocks;
     int clusters = ctx->num_sms / 2;
     if (clusters > tiles) clusters = tiles;
-    kern<<<2 * clusters, C::kThreads, C::kSmem, ctx->stream>>>(a);
+    gemm_pair_kernel<<<2 * clusters, kPairThreads, kPairSmem, ctx->stream>>>(a);
     return cudaGetLastError();
 }
 
 }  // namespace
 
-int w4_gemm_mode() {
-    static const int mode = [] {
-        const char *e = getenv("TCE_W4_GEMM");
-        if (!e) return (int)W4G_PAIR_OVERLAP;  // measured best on B200 (profiles/README.md): CTA-pair GEMM, expansion of the next linear overlapped
-        const std::string v(e);
-        if (v == "fused") return (int)W4G_FUSED;
-        if (v == "pair") return (int)W4G_PAIR;
-        if (v == "pair_fused") return (int)W4G_PAIR_FUSED;
-        if (v == "pair_overlap") return (int)W4G_PAIR_OVERLAP;
-        if (v == "expand") return (int)W4G_EXPAND;
-        return (int)W4G_PAIR_OVERLAP;
-    }();
-    return mode;
+cudaError_t w4_scratch_reserve(Ctx *ctx, size_t elems) {
+    if (ctx->w16_scratch_elems >= elems) return cudaSuccess;
+    if (ctx->w16_scratch) {  // rare: grows to the largest weight matrix seen (cudaFree synchronises)
+        cudaError_t e = cudaFree(ctx->w16_scratch);
+        ctx->w16_scratch = nullptr;
+        ctx->w16_scratch_elems = 0;
+        if (e != cudaSuccess) return e;
+    }
+    cudaError_t e = cudaMalloc(&ctx->w16_scratch, elems * sizeof(__half));
+    if (e == cudaSuccess) ctx->w16_scratch_elems = elems;
+    return e;
+}
+
+cudaError_t launch_w4_expand(Ctx *ctx, const uint32_t *w, const uint32_t *zeros, const __half *scales, __half *out, int OC, int IC) {
+    const int wpr = IC / 8, zw = zeros_width(IC, kW4Group);
+    const long long n = (long long)OC * wpr;
+    w4_expand_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(w, zeros, scales, out, OC, wpr, zw, zw * 8);
+    return cudaGetLastError();
 }
 
 // W fp16 [N][K] (ldw elements between rows)
@@ -497,7 +391,7 @@ cudaError_t launch_gemm_f16_pair(Ctx *ctx, const __half *X, long long ldx, const
     a.C = C;
     a.ldc = ldc;
     a.add_f32 = add_f32;
-    return launch_pair<false>(ctx, a);
+    return launch_pair(ctx, a);
 }
 
 // act[M][F] = SiLU(X Wg^T) * (X Wu^T), W = fp16 [2F][K] with the gate rows first; F % 128 == 0, ldc % 8 == 0
@@ -514,38 +408,7 @@ cudaError_t launch_gemm_f16_pair_silu(Ctx *ctx, const __half *X, long long ldx, 
     a.ldc = ldc;
     a.pn = kPairN;
     a.silu_F = F;
-    return launch_pair<false>(ctx, a);
-}
-
-// W packed QM_CUDA int4
-cudaError_t launch_gemm_w4_pair(Ctx *ctx, const __half *X, long long ldx, const uint32_t *w, const uint32_t *zeros, const __half *scales, void *C, long long ldc,
-                                int M, int N, int K, int add_f32) {
-    if (M < 1 || N < 1 || K < 128 || (K % 128) || (ldx % 8) || !encoder2()) return cudaErrorInvalidValue;
-    PairArgs a = {};
-    if (!encode_f16(&a.tmA, X, M, K, ldx)) return cudaErrorInvalidValue;
-    {
-        const cuuint64_t gdim[2] = {(cuuint64_t)(K / 8), (cuuint64_t)N};
-        const cuuint64_t gstride[1] = {(cuuint64_t)(K / 8) * 4};
-        const cuuint32_t box[2] = {8u, (cuuint32_t)kHalfN};
-        const cuuint32_t estr[2] = {1, 1};
-        if (encoder2()(&a.tmB, CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, const_cast<uint32_t *>(w), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                       CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-            return cudaErrorInvalidValue;
-    }
-    a.scales = scales;
-    a.zeros = zeros;
-    a.zeros_w = zeros_width(K, kW4Group);
-    a.sf_w = a.zeros_w * 8;
-    a.M = M;
-    a.N = N;
-    a.k_blocks = K / 64;
-    a.m_blocks = (M + 255) / 256;
-    a.n_blocks = (N + kPairN - 1) / kPairN;
-    a.pn = kPairN;
-    a.C = C;
-    a.ldc = ldc;
-    a.add_f32 = add_f32;
-    return launch_pair<true>(ctx, a);
+    return launch_pair(ctx, a);
 }
 
 }  // namespace tce

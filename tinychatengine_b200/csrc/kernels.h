@@ -111,20 +111,11 @@ cudaError_t encode_w4_tmap_units(CUtensorMap *out, const void *w, int rows, int 
 cudaError_t launch_naive_fp16_int4(Ctx *ctx, const __half *A, const int32_t *B, const __half *scales, __half *C, int M, int IC, int OC, int block);
 cudaError_t launch_f32_matmul_transposed(Ctx *ctx, const float *A, const float *B, float *C, int M, int N, int K);
 
+// W4A16 prefill GEMM (gemm_tc2.cu): the int4 weights are expanded to fp16 (launch_w4_expand), then multiplied on CTA pairs
+// (tcgen05.mma.cta_group::2, 256 x 256 tiles)
 cudaError_t launch_w4_expand(Ctx *ctx, const uint32_t *w, const uint32_t *zeros, const __half *scales, __half *out, int OC, int IC);
-cudaError_t launch_gemm_f16_tc(Ctx *ctx, const __half *A, long long lda, const __half *B, long long ldb, void *C, long long ldc, int M, int N, int K,
-                               int add_f32 = 0);
-// fused variant (gemm_w4_tc.cu): the nibbles are unpacked inside the tile pipeline, no fp16 copy of the weights in HBM
-cudaError_t launch_gemm_w4_tc(Ctx *ctx, const __half *X, long long ldx, const uint32_t *w, const uint32_t *zeros, const __half *scales, void *C, long long ldc,
-                              int M, int N, int K, int add_f32);
-// which W4A16 large-M GEMM runs (TCE_W4_GEMM=expand|fused|pair|pair_fused; the default is the measured best, profiles/README.md)
-enum W4GemmMode : int { W4G_EXPAND = 0, W4G_FUSED = 1, W4G_PAIR = 2, W4G_PAIR_FUSED = 3, W4G_PAIR_OVERLAP = 4 };
-int w4_gemm_mode();
-// CTA-pair variants (gemm_tc2.cu): tcgen05.mma.cta_group::2 on 256 x 256 tiles, W as fp16 or as packed int4 (unpack fused)
 cudaError_t launch_gemm_f16_pair(Ctx *ctx, const __half *X, long long ldx, const __half *W, long long ldw, void *C, long long ldc, int M, int N, int K, int add_f32);
 cudaError_t launch_gemm_f16_pair_silu(Ctx *ctx, const __half *X, long long ldx, const __half *W, long long ldw, __half *act, long long ldc, int M, int F, int K);
-cudaError_t launch_gemm_w4_pair(Ctx *ctx, const __half *X, long long ldx, const uint32_t *w, const uint32_t *zeros, const __half *scales, void *C, long long ldc,
-                                int M, int N, int K, int add_f32);
 cudaError_t w4_scratch_reserve(Ctx *ctx, size_t elems);  // grows ctx->w16_scratch (may synchronise the device)
 
 // host-side mirror of the stream-K partition used by the kernel (unit-tested on the CPU)

@@ -446,7 +446,7 @@ cudaError_t LlamaDecoder::build_persistent(std::string *err) {
         o.epi = epi;
         return o;
     };
-    // TMA box plans (odd box widths, see persistent.h) and the distinct widths each op needs a tensor map for
+    // TMA box plans (see make_box_plan) and the distinct widths each op needs a tensor map for
     int widths[pk::OPI_COUNT][pk::kMapsPerMat] = {}, nwidths[pk::OPI_COUNT] = {};
     const bool tp = tp_ > 1;
     a.op[pk::OPI_QKV] = mk(E, (H + 2 * KVH) * hd, 3, 0, H * hd, KVH * hd, pk::PX_RMS_F32, pk::PE_HALF_LL);
@@ -461,9 +461,9 @@ cudaError_t LlamaDecoder::build_persistent(std::string *err) {
         a.op[i].plan[1] = (NG > pk::kStageGroups && rem) ? pk::make_box_plan(rem, widths[i], &nwidths[i]) : a.op[i].plan[0];
         for (int k = 0; k < pk::kMaxBoxes; k++)
             if ((k < a.op[i].plan[0].nbox && a.op[i].plan[0].map[k] < 0) || (k < a.op[i].plan[1].nbox && a.op[i].plan[1].map[k] < 0)) return no("too many box widths");
-        // unit boxes ([group][row][64 B], conflict-free LDS.128) where the dense consumer applies (every stage made of 16-group boxes)
-        static const bool want_units = !getenv("TCE_PK_UNIT_BOXES") || atoi(getenv("TCE_PK_UNIT_BOXES")) != 0;  // default on: +1.3 % (profiles/README.md)
-        a.op[i].unit = (want_units && a.op[i].plan[0].bw[0] == 16 && (NG & 15) == 0) ? 1 : 0;
+        // unit boxes ([group][row][64 B], conflict-free LDS.128: +1.3 %, profiles/README.md) where the dense consumer applies (every stage made
+        // of 16-group boxes)
+        a.op[i].unit = (a.op[i].plan[0].bw[0] == 16 && (NG & 15) == 0) ? 1 : 0;
         if (a.op[i].IC > max_ic) max_ic = a.op[i].IC;
         if (a.op[i].NG > max_ng) max_ng = a.op[i].NG;
         if (a.op[i].IC % kW4Group || a.op[i].num_tiles < 1) return no("bad GEMV shape");
@@ -476,14 +476,8 @@ cudaError_t LlamaDecoder::build_persistent(std::string *err) {
     a.max_ng = max_ng;
     a.E = E;
     a.nst = pk::pick_stages(ctx_->smem_optin, xs, max_ng, E);
-    if (getenv("TCE_PK_STAGES")) {
-        const int want = atoi(getenv("TCE_PK_STAGES"));
-        if (want >= 2 && want < a.nst) a.nst = want;
-    }
     if (a.nst < 2) return no("shared memory too small for the persistent kernel");
-    a.l2_prefetch = getenv("TCE_PK_L2_PREFETCH") ? atoi(getenv("TCE_PK_L2_PREFETCH")) : 0;
     a.pair = 0;  // decided below, once the shared-memory footprint is known
-    if (getenv("TCE_PK_POLL_NS")) DCK(pk::set_poll_backoff((unsigned)atoi(getenv("TCE_PK_POLL_NS"))));
 
     auto dalloc = [&](size_t bytes) -> void * {
         void *p = nullptr;
@@ -865,49 +859,23 @@ cudaError_t LlamaDecoder::prefill_reserve(int n) {
     return cudaSuccess;
 }
 
-// C[n][sum oc] (row-major, leading dimension ldc) = X[n][ic] * [deq(t0); deq(t1); ...]^T : the `count` weight matrices (same ic) are
-// expanded into consecutive row ranges of the fp16 scratch and multiplied by ONE GEMM (q|k|v and gate|up share their input)
+// C[n][sum oc] (row-major, leading dimension ldc) = X[n][ic] * [deq(t0); deq(t1); ...]^T : the `count` weight matrices (same ic) of the
+// prompt pass's next job were expanded into consecutive row ranges of one fp16 scratch half, and ONE GEMM multiplies them (q|k|v and
+// gate|up share their input).  Called in the order of pf_jobs_.
 cudaError_t LlamaDecoder::prefill_linear(const tce_w4_tensor *const *ts, int count, const __half *x, void *C, long long ldc, int n, bool add_f32, bool silu) {
     const int ic = ts[0]->ic;
-    const int mode = w4_gemm_mode();
-    if (mode == W4G_FUSED || mode == W4G_PAIR_FUSED) {
-        // one launch per tensor, each writing its column range of C: the packed weights are unpacked inside the GEMM's tile pipeline
-        size_t c0 = 0;
-        for (int i = 0; i < count; i++) {
-            const tce_w4_tensor &t = *ts[i];
-            void *Ci = add_f32 ? static_cast<void *>(static_cast<float *>(C) + c0) : static_cast<void *>(static_cast<__half *>(C) + c0);
-            if (mode == W4G_PAIR_FUSED)
-                DCK(launch_gemm_w4_pair(ctx_, x, ic, (const uint32_t *)t.w, (const uint32_t *)t.zeros, (const __half *)t.scales, Ci, ldc, n, t.oc, ic, add_f32 ? 1 : 0));
-            else
-                DCK(launch_gemm_w4_tc(ctx_, x, ic, (const uint32_t *)t.w, (const uint32_t *)t.zeros, (const __half *)t.scales, Ci, ldc, n, t.oc, ic, add_f32 ? 1 : 0));
-            c0 += (size_t)t.oc;
-        }
-        return cudaSuccess;
-    }
     size_t rows = 0;
     for (int i = 0; i < count; i++) rows += (size_t)ts[i]->oc;
-    if (mode == W4G_PAIR_OVERLAP && !pf_jobs_.empty()) {
-        // this job's weights were expanded on the side stream while the previous GEMM ran; queue the next job's expansion, then run
-        const int j = pf_next_job_++;
-        const int b = j & 1;
-        if (j + 1 < (int)pf_jobs_.size()) DCK(pf_expand_job(j + 1));
-        DCK(cudaStreamWaitEvent(ctx_->stream, pf_expanded_[b], 0));
-        if (silu)
-            DCK(launch_gemm_f16_pair_silu(ctx_, x, ic, pf_w16_[b], ic, (__half *)C, ldc, n, (int)(rows / 2), ic));
-        else
-            DCK(launch_gemm_f16_pair(ctx_, x, ic, pf_w16_[b], ic, C, ldc, n, (int)rows, ic, add_f32 ? 1 : 0));
-        return cudaEventRecord(pf_consumed_[b], ctx_->stream);
-    }
-    DCK(w4_scratch_reserve(ctx_, rows * ic));
-    size_t r0 = 0;
-    for (int i = 0; i < count; i++) {
-        const tce_w4_tensor &t = *ts[i];
-        DCK(launch_w4_expand(ctx_, (const uint32_t *)t.w, (const uint32_t *)t.zeros, (const __half *)t.scales, ctx_->w16_scratch + r0 * ic, t.oc, ic));
-        r0 += (size_t)t.oc;
-    }
-    if (silu) return launch_gemm_f16_pair_silu(ctx_, x, ic, ctx_->w16_scratch, ic, (__half *)C, ldc, n, (int)(rows / 2), ic);
-    if (mode == W4G_PAIR || mode == W4G_PAIR_OVERLAP) return launch_gemm_f16_pair(ctx_, x, ic, ctx_->w16_scratch, ic, C, ldc, n, (int)rows, ic, add_f32 ? 1 : 0);
-    return launch_gemm_f16_tc(ctx_, x, ic, ctx_->w16_scratch, ic, C, ldc, n, (int)rows, ic, add_f32 ? 1 : 0);
+    // this job's weights were expanded on the side stream while the previous GEMM ran; queue the next job's expansion, then run
+    const int j = pf_next_job_++;
+    const int b = j & 1;
+    if (j + 1 < (int)pf_jobs_.size()) DCK(pf_expand_job(j + 1));
+    DCK(cudaStreamWaitEvent(ctx_->stream, pf_expanded_[b], 0));
+    if (silu)
+        DCK(launch_gemm_f16_pair_silu(ctx_, x, ic, pf_w16_[b], ic, (__half *)C, ldc, n, (int)(rows / 2), ic));
+    else
+        DCK(launch_gemm_f16_pair(ctx_, x, ic, pf_w16_[b], ic, C, ldc, n, (int)rows, ic, add_f32 ? 1 : 0));
+    return cudaEventRecord(pf_consumed_[b], ctx_->stream);
 }
 
 // expansion of job j into scratch half (j & 1) on the side stream, after the GEMM that last read that half
@@ -936,35 +904,33 @@ cudaError_t LlamaDecoder::prefill(const int *tokens_host, int n, int pos0, float
     for (int i = 0; i < n; i++)
         if (tokens_host[i] < 0 || tokens_host[i] >= cfg_.vocab_size) return cudaErrorInvalidValue;
     DCK(prefill_reserve(n));
-    if (w4_gemm_mode() == W4G_PAIR_OVERLAP) {
-        if (pf_jobs_.empty()) {
-            size_t need = 0;
-            for (int l = 0; l < cfg_.num_layers; l++) {
-                const tce_llama_layer &L = layers_[l];
-                pf_jobs_.push_back(PfJob{{&L.q, &L.k, &L.v}, 3});
-                pf_jobs_.push_back(PfJob{{&L.o, nullptr, nullptr}, 1});
-                pf_jobs_.push_back(PfJob{{&L.gate, &L.up, nullptr}, 2});
-                pf_jobs_.push_back(PfJob{{&L.down, nullptr, nullptr}, 1});
-            }
-            for (const PfJob &jb : pf_jobs_) {
-                size_t e = 0;
-                for (int i = 0; i < jb.count; i++) e += (size_t)jb.ts[i]->oc * jb.ts[i]->ic;
-                need = e > need ? e : need;
-            }
-            for (int b = 0; b < 2; b++) {
-                DCK(cudaMalloc((void **)&pf_w16_[b], need * sizeof(__half)));
-                DCK(cudaEventCreateWithFlags(&pf_expanded_[b], cudaEventDisableTiming));
-                DCK(cudaEventCreateWithFlags(&pf_consumed_[b], cudaEventDisableTiming));
-            }
-            pf_w16_elems_ = need;
-            DCK(cudaStreamCreateWithFlags(&pf_side_, cudaStreamNonBlocking));
+    if (pf_jobs_.empty()) {
+        size_t need = 0;
+        for (int l = 0; l < cfg_.num_layers; l++) {
+            const tce_llama_layer &L = layers_[l];
+            pf_jobs_.push_back(PfJob{{&L.q, &L.k, &L.v}, 3});
+            pf_jobs_.push_back(PfJob{{&L.o, nullptr, nullptr}, 1});
+            pf_jobs_.push_back(PfJob{{&L.gate, &L.up, nullptr}, 2});
+            pf_jobs_.push_back(PfJob{{&L.down, nullptr, nullptr}, 1});
         }
-        pf_next_job_ = 0;
-        // the side stream starts after everything already queued on the main stream (a previous prompt's GEMMs read the scratch)
-        DCK(cudaEventRecord(pf_consumed_[0], ctx_->stream));
-        DCK(cudaStreamWaitEvent(pf_side_, pf_consumed_[0], 0));
-        DCK(pf_expand_job(0));
+        for (const PfJob &jb : pf_jobs_) {
+            size_t e = 0;
+            for (int i = 0; i < jb.count; i++) e += (size_t)jb.ts[i]->oc * jb.ts[i]->ic;
+            need = e > need ? e : need;
+        }
+        for (int b = 0; b < 2; b++) {
+            DCK(cudaMalloc((void **)&pf_w16_[b], need * sizeof(__half)));
+            DCK(cudaEventCreateWithFlags(&pf_expanded_[b], cudaEventDisableTiming));
+            DCK(cudaEventCreateWithFlags(&pf_consumed_[b], cudaEventDisableTiming));
+        }
+        pf_w16_elems_ = need;
+        DCK(cudaStreamCreateWithFlags(&pf_side_, cudaStreamNonBlocking));
     }
+    pf_next_job_ = 0;
+    // the side stream starts after everything already queued on the main stream (a previous prompt's GEMMs read the scratch)
+    DCK(cudaEventRecord(pf_consumed_[0], ctx_->stream));
+    DCK(cudaStreamWaitEvent(pf_side_, pf_consumed_[0], 0));
+    DCK(pf_expand_job(0));
     cudaStream_t s = ctx_->stream;
     const int E = cfg_.embed_dim, F = cfg_.hidden_dim, H = cfg_.num_heads, KVH = cfg_.num_kv_heads, hd = cfg_.head_dim;
     const long long Q = (long long)(H + 2 * KVH) * hd;
@@ -992,8 +958,7 @@ cudaError_t LlamaDecoder::prefill(const int *tokens_host, int n, int pos0, float
         DCK(launch_attn_prefill(ctx_, a));
         DCK(prefill_linear(o1, 1, pf_att_, pf_x_, E, n, true));  // residual add in the GEMM epilogue
         DCK(launch_rmsnorm_rows_f32(ctx_, pf_x_, L.post_norm, pf_xn_, n, E, cfg_.rms_eps));
-        const int gm = w4_gemm_mode();
-        if ((gm == W4G_PAIR || gm == W4G_PAIR_OVERLAP) && (F % 128) == 0) {
+        if ((F % 128) == 0) {
             DCK(prefill_linear(gu, 2, pf_xn_, pf_act_, F, n, false, true));  // SiLU(gate) * up in the GEMM epilogue: gate|up never reach HBM
         } else {
             DCK(prefill_linear(gu, 2, pf_xn_, pf_gu_, 2LL * F, n, false));

@@ -96,8 +96,8 @@ class LlamaDecoder {
     __half *pf_gu_ = nullptr;       // [n][2F] gate | up
     __half *pf_act_ = nullptr;      // [n][F]
     int *pf_tok_ = nullptr;
-    // W4G_PAIR_OVERLAP: the int4 -> fp16 expansion of the NEXT linear runs on a side stream into the other half of a double-buffered scratch
-    // while the tensor cores work on the current one (the expansion is HBM-bound, the GEMM tensor-bound)
+    // the int4 -> fp16 expansion of the NEXT linear runs on a side stream into the other half of a double-buffered scratch while the
+    // tensor cores work on the current one (the expansion is HBM-bound, the GEMM tensor-bound)
     __half *pf_w16_[2] = {nullptr, nullptr};
     size_t pf_w16_elems_ = 0;
     cudaStream_t pf_side_ = nullptr;

@@ -12,7 +12,7 @@ namespace tce {
 namespace pk {
 
 constexpr int kCW = 16;                          // consumer warps
-constexpr int kAuxWarps = 4;                     // warpgroup 0: loader warp, epilogue warp, L2-prefetch warp, one spare warp that only donates its registers
+constexpr int kAuxWarps = 4;                     // warpgroup 0: loader warp, epilogue warp, two spare warps that only donate their registers
 constexpr int kThreads = 32 * (kAuxWarps + kCW); // 640
 constexpr int kConsumerThreads = 32 * kCW;       // 512
 constexpr int kStageGroups = 32;                 // 128-k groups per ring stage: every consumer warp owns two of them
@@ -33,7 +33,7 @@ enum Epi : int { PE_HALF_LL = 0, PE_DELTA_LL = 1, PE_SILU_LL = 2, PE_LOGITS = 3 
 enum OpIdx : int { OPI_QKV = 0, OPI_O = 1, OPI_GATEUP = 2, OPI_DOWN = 3, OPI_LMHEAD = 4, OPI_COUNT = 5 };
 
 // shape of one GEMV op; identical for every layer, so it lives in the kernel parameter block
-// A stage's <= 32 groups arrive as up to four 2-D TMA boxes (by default two dense boxes of 16 groups; see make_box_plan).
+// A stage's <= 32 groups arrive as one or two dense TMA boxes of up to 16 groups (see make_box_plan).
 struct BoxPlan {
     int nbox;
     int b0[kMaxBoxes];   // first group of the box within the stage
@@ -88,7 +88,6 @@ struct Args {
     int H, KVH, nrep, max_ctx, E, V, F;
     int nsplit_max;
     int nst;                     // ring depth
-    int l2_prefetch;             // 1: a second producer warp prefetches the stages into L2 ahead of the loader
     int pair;                    // 1: launched as clusters of two CTAs that share the activation staging: each polls and quantises every other
                                  // 128-group and mirrors the result into its partner's shared memory (st.async over DSMEM)
     int xs_bytes;                // activation-plane buffer (also the attention scratch)
@@ -107,12 +106,11 @@ int pick_stages(int smem_optin, int xs_bytes, int max_ng, int E);
 int attn_scratch_bytes(int nrep);
 int attn_nsplit_max(int ncta, int KVH, int max_ctx);
 cudaError_t launch(Ctx *ctx, const Args &a, cudaStream_t stream);
-bool pair_supported(Ctx *ctx, const Args &a);
-cudaError_t set_poll_backoff(unsigned ns);  // pause of a failed hand-off poll before it asks L2 again (default 100 ns)  // the grid fits as co-resident clusters of two CTAs
+bool pair_supported(Ctx *ctx, const Args &a);  // the grid fits as co-resident clusters of two CTAs
 // one-off repack of a (possibly multi-segment / gate-up paired) matrix's scales and zeros into per-stage records
 cudaError_t repack_meta(Ctx *ctx, const W4Seg *segs, int nseg, int pair, int IC, uint8_t *out, cudaStream_t stream);
 cudaError_t encode_kv_tmap(CUtensorMap *out, const void *kv, long long rows);
-// split n <= 32 groups into odd-width boxes; `widths` collects the distinct widths (<= kMapsPerMat) of the op
+// split n <= 32 groups into dense boxes of at most 16 groups; `widths` collects the distinct widths (<= kMapsPerMat) of the op
 BoxPlan make_box_plan(int n, int *widths, int *nwidths);
 
 }  // namespace pk

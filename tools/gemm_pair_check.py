@@ -1,10 +1,9 @@
 #!/usr/bin/env python
-"""Check + time one W4A16 large-M GEMM variant (TCE_W4_GEMM=expand|fused|pair|pair_fused, read once per process) against a torch fp32
-reference of the dequantised weights: a few ragged shapes for correctness, the Llama-2-13B prefill shapes for speed.
-    TCE_W4_GEMM=pair_fused python tools/gemm_pair_check.py
+"""Check + time the W4A16 large-M GEMM (tce_w4a16_gemm: int4 -> fp16 expansion + CTA-pair tcgen05 GEMM) against a torch fp32 reference
+of the dequantised weights: a few ragged shapes for correctness, the Llama-2-13B prefill shapes for speed.
+    python tools/gemm_pair_check.py
 """
 import json
-import os
 import sys
 from pathlib import Path
 
@@ -25,7 +24,6 @@ def dequant(w, z, s, ic):
 
 
 def main():
-    mode = os.environ.get("TCE_W4_GEMM", "expand")
     dev = torch.device("cuda", 0)
     ctx = Context(0)
     ok = True
@@ -37,7 +35,7 @@ def main():
         err = float((y - ref).abs().max() / ref.abs().max())
         good = err < 2e-3
         ok &= good
-        print(json.dumps({"mode": mode, "check": [m, oc, ic], "rel_err": err, "ok": good}), flush=True)
+        print(json.dumps({"check": [m, oc, ic], "rel_err": err, "ok": good}), flush=True)
     if not ok:
         raise SystemExit(1)
     M = 2048
@@ -56,7 +54,7 @@ def main():
         e1.record()
         torch.cuda.synchronize()
         t = e0.elapsed_time(e1) / 10 * 1e-3
-        print(json.dumps({"mode": mode, "shape": name, "M": M, "ms": round(t * 1e3, 4), "tflops": round(2.0 * M * oc * ic / t / 1e12, 1)}), flush=True)
+        print(json.dumps({"shape": name, "M": M, "ms": round(t * 1e3, 4), "tflops": round(2.0 * M * oc * ic / t / 1e12, 1)}), flush=True)
 
 
 if __name__ == "__main__":

@@ -1,5 +1,5 @@
-"""Target for `ncu -k regex:gemm_pair`: four W4A16 GEMM calls at the Llama-2-13B q|k|v prefill shape (M = 2048, 15360 x 5120) through tce_w4a16_gemm;
-select the variant with TCE_W4_GEMM=expand|fused|pair|pair_fused.  See profiles/README.md (prefill section)."""
+"""Target for `ncu -k regex:gemm_pair`: four W4A16 GEMM calls at the Llama-2-13B q|k|v prefill shape (M = 2048, 15360 x 5120) through tce_w4a16_gemm
+(int4 -> fp16 expansion + the CTA-pair GEMM).  See profiles/README.md (prefill section)."""
 import sys, torch
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
